@@ -265,6 +265,24 @@ def dist_setup(n_gpus):
     return rank, world, local, dist
 
 
+DUMP_SAMPLE = 1 << 22   # values sampled from each dumped output: 2 x 4 Mi float32 = 32 MiB
+
+
+def dump_outputs(out_dir, packed, big, ids_dev):
+    """What the timed path computed in its last step, so that two builds can be compared output for output: the packed
+    buffer the gather kernel wrote (packed.npy) and the pool pages the scatter kernel wrote back (pool.npy).  Both are
+    ~21 GB, so each is a sample at fixed seeded byte positions, stored as float32 (the bytes are exact in it)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(2024)
+    pos = torch.from_numpy(np.sort(rng.integers(0, packed.numel(), DUMP_SAMPLE))).cuda()
+    np.save(os.path.join(out_dir, "packed.npy"), packed[pos].float().cpu().numpy())
+    t = torch.from_numpy(rng.integers(0, big.shape[0], DUMP_SAMPLE)).cuda()
+    k = torch.from_numpy(rng.integers(0, ids_dev.numel(), DUMP_SAMPLE)).cuda()
+    b = torch.from_numpy(rng.integers(0, big.shape[2], DUMP_SAMPLE)).cuda()
+    np.save(os.path.join(out_dir, "pool.npy"), big[t, ids_dev[k], b].float().cpu().numpy())
+
+
 def workload_config(n_gpus, blocks_per_step=N_BLOCKS):
     cfg = {"workload": "BASELINE config #2: Llama-3-8B fp16 paged-KV, 16-tok blocks, save+load 10k blocks GPU<->host",
            "tensors": T_TENSORS, "fragment_bytes": FRAG_BYTES, "block_bytes": BLOCK_BYTES, "pool_blocks": POOL_BLOCKS,
@@ -482,6 +500,8 @@ def run_ours(args):
     dev_ms = max_over_ranks(dist, start.elapsed_time(stop))
     gather_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in ev_sets]))
     scatter_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in ev_sets]))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, packed, big, ids_dev)
     # untimed proof that the load leg really restores: save, ZERO every saved page, load, compare
     sum0 = pool_checksum(big)
     pool.gather_dev(ids_dev, packed)
@@ -809,7 +829,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-migration", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip configs #1/#3/#5, ingest and manager lookup (ncu captures)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of what the last step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -5,6 +5,7 @@ import math
 import os
 import shutil
 import struct
+import tempfile
 import time
 
 import numpy as np
@@ -14,7 +15,8 @@ from oracle import offload_oracle as oo
 
 pytestmark = pytest.mark.gpu
 
-TMP_DIR = "/tmp/kvb-shared-kv-test"
+# one directory per test process: on a machine shared by several users a fixed name may belong to someone else
+TMP_DIR = os.path.join(tempfile.gettempdir(), f"kvb-shared-kv-test-{os.getpid()}")
 
 
 def _kv_tensors(torch, num_layers, num_blocks, block_size, num_heads, head_size, dtype, seed=42):
