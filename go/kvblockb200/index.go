@@ -138,6 +138,40 @@ func (ix *Index) Evict(_ context.Context, key kvblock.BlockHash, keyType kvblock
 	return nil
 }
 
+// RemovePods removes every entry of the named pods (of the named tiers; none = every tier) from every key in one device
+// sweep (kvb_index_remove_pods).  No reference counterpart: the reference ignores AllBlocksCleared (pool.go:388-395).
+// Keys left empty are deleted, no key's recency changes, the engine-key map is untouched.  Names the index has never
+// seen match nothing.  Returns (entries removed, keys deleted).
+func (ix *Index) RemovePods(_ context.Context, pods []string, tiers []string) (int64, int64, error) {
+	ix.mu.Lock()
+	defer ix.mu.Unlock()
+	var pids []C.uint16_t
+	for _, name := range pods {
+		if id, ok := ix.pods[name]; ok {
+			pids = append(pids, C.uint16_t(id))
+		}
+	}
+	var tids []C.uint8_t
+	for _, name := range tiers {
+		if id, ok := ix.tiers[name]; ok {
+			tids = append(tids, C.uint8_t(id))
+		}
+	}
+	if len(pids) == 0 || (len(tiers) > 0 && len(tids) == 0) {
+		return 0, 0, nil
+	}
+	var tp *C.uint8_t
+	if len(tids) > 0 {
+		tp = &tids[0]
+	}
+	var removed, deleted C.int64_t
+	if rc := C.kvb_index_remove_pods(ix.h, &pids[0], C.int32_t(len(pids)), tp, C.int32_t(len(tids)), &removed,
+		&deleted); rc != 0 {
+		return 0, 0, lastError(rc)
+	}
+	return int64(removed), int64(deleted), nil
+}
+
 // GetRequestKey mirrors in_memory.go:298-304.
 func (ix *Index) GetRequestKey(_ context.Context, engineKey kvblock.BlockHash) (kvblock.BlockHash, error) {
 	var out C.uint64_t

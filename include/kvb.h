@@ -247,6 +247,8 @@ int64_t kvb_index_num_keys(kvb_index_t* idx);
 #define KVB_EVENT_BLOCK_STORED 0
 #define KVB_EVENT_BLOCK_REMOVED 1
 #define KVB_EVENT_OTHER 2 /* AllBlocksCleared / unknown: ignored, as in the reference (pool.go:388-395) */
+#define KVB_EVENT_POD_CLEARED 3 /* remove entry.pod's entries of entry.tier (kvb_index_remove_pods; opt-in AllBlocksCleared).
+                                   Applied at its place among the round's non-stored events: what is queued goes first */
 typedef struct kvb_kv_event {
   int32_t type;               /* KVB_EVENT_* */
   int32_t stream;             /* ordering domain: the pod */
@@ -259,6 +261,19 @@ typedef struct kvb_kv_event {
 } kvb_kv_event_t;
 int kvb_index_ingest_events(kvb_index_t* idx, const kvb_kv_event_t* events, int32_t n_events, const uint32_t* tokens,
                             const uint64_t* engine_keys, int32_t block_size, int32_t* out_skipped);
+
+/* Remove every entry of `pods` (interned ids, n_pods >= 1) from every key; tiers == NULL / n_tiers == 0: every tier,
+ * otherwise an entry goes only if its tier is listed too.  The speculative bit is not looked at.  No reference
+ * counterpart (pool.go:388-395 ignores AllBlocksCleared): one device sweep over the whole table, since only the table
+ * knows which request keys hold a pod.
+ *   - surviving entries keep their inner-LRU order; a key left empty is deleted (in_memory.go:281-292)
+ *   - no recency stamp changes (a sequence of Evict calls would refresh every key it touches); the engine-key map is
+ *     untouched, as Evict(RequestKey) leaves it
+ *   - queued Add / Evict ops are applied first, ops queued later come after: the result is that of call order
+ *   - ids never interned simply match nothing
+ * out_entries_removed / out_keys_deleted may be NULL. */
+int kvb_index_remove_pods(kvb_index_t* idx, const uint16_t* pods, int32_t n_pods, const uint8_t* tiers, int32_t n_tiers,
+                          int64_t* out_entries_removed, int64_t* out_keys_deleted);
 
 /* apply the queued Add / Evict operations to the device table and wait for it (reads do this implicitly) */
 int kvb_index_flush(kvb_index_t* idx, void* stream);

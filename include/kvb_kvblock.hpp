@@ -4,7 +4,7 @@
 // C ABI is provided in C++ with the SAME names, argument meaning and error behaviour as the Go interfaces:
 //
 //   kvblock::TokenProcessor   pkg/kvcache/kvblock/token_processor.go:55-69   (TokensToKVBlockKeys, BlockSize)
-//   kvblock::Index            pkg/kvcache/kvblock/index.go:120-149           (Lookup, Add, Evict, GetRequestKey)
+//   kvblock::Index            pkg/kvcache/kvblock/index.go:120-149           (Lookup, Add, Evict, GetRequestKey; RemovePods)
 //   kvblock::PodEntry, BlockHash, KeyType, BlockExtraFeatures, MMHash         index.go:152-183, extra_keys.go:26-34
 //   kvcache::Indexer          pkg/kvcache/indexer.go:65-304                   (ScoreTokens, ComputeBlockKeysFromTokens)
 //
@@ -22,6 +22,7 @@
 #include <stdexcept>
 #include <string>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "kvb.h"
@@ -229,6 +230,28 @@ class Index {
     std::lock_guard<std::mutex> lk(mu_);
     auto e = intern(entries);
     check(kvb_index_evict(h_, key, (int)keyType, e.data(), (int32_t)e.size()));
+  }
+  // Every entry of `pods` (of `tiers`; empty = every tier) leaves every key, in one device sweep (kvb_index_remove_pods).
+  // No reference counterpart (pool.go:388-395 ignores AllBlocksCleared).  Keys left empty are deleted, no recency
+  // changes, the engine-key map is untouched; names the index has never seen match nothing.
+  // Returns {entries removed, keys deleted}.
+  std::pair<int64_t, int64_t> RemovePods(const std::vector<std::string>& pods, const std::vector<std::string>& tiers = {}) {
+    std::lock_guard<std::mutex> lk(mu_);
+    std::vector<uint16_t> p;
+    for (const auto& name : pods) {
+      auto it = pods_.find(name);
+      if (it != pods_.end()) p.push_back(it->second);
+    }
+    std::vector<uint8_t> t;
+    for (const auto& name : tiers) {
+      auto it = tiers_.find(name);
+      if (it != tiers_.end()) t.push_back(it->second);
+    }
+    if (p.empty() || (!tiers.empty() && t.empty())) return {0, 0};
+    int64_t removed = 0, deleted = 0;
+    check(kvb_index_remove_pods(h_, p.data(), (int32_t)p.size(), t.empty() ? nullptr : t.data(), (int32_t)t.size(),
+                                &removed, &deleted));
+    return {removed, deleted};
   }
   // GetRequestKey (in_memory.go:298-304)
   BlockHash GetRequestKey(BlockHash engineKey) {

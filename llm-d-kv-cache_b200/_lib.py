@@ -56,7 +56,7 @@ class KvEvent(C.Structure):  # kvb_kv_event_t
                 ("root_hash", C.c_uint64), ("entry", PodEntryC), ("pad", C.c_int32)]
 
 
-EVENT_BLOCK_STORED, EVENT_BLOCK_REMOVED, EVENT_OTHER = 0, 1, 2
+EVENT_BLOCK_STORED, EVENT_BLOCK_REMOVED, EVENT_OTHER, EVENT_POD_CLEARED = 0, 1, 2, 3
 
 
 class IpcMem(C.Structure):
@@ -107,6 +107,7 @@ SIGNATURES = {
     "kvb_index_get_request_key": (C.c_int, [_vp, _u64, _P(_u64)]),
     "kvb_index_num_keys": (_i64, [_vp]),
     "kvb_index_ingest_events": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i32, _P(_i32)]),
+    "kvb_index_remove_pods": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _P(_i64), _P(_i64)]),
     "kvb_index_flush": (C.c_int, [_vp, _vp]),
     "kvb_index_get_stats": (C.c_int, [_vp, _P(IndexStats)]),
     "kvb_index_lookup": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp, _vp, _P(_i64)]),

@@ -68,6 +68,7 @@ struct Counters {  // device resident
   unsigned long long live, tombs, order_head, evicted, inserted, removed, stale_skipped, scans;
   long long resume_at;            // sequential replay: first op not yet applied, -1 when the batch is done
   unsigned long long pending_evict;  // an eviction the replay still owes (its order array ran out)
+  unsigned long long purge_entries, purge_keys;  // pod removal: entries removed / keys deleted by the last sweep
 };
 
 struct TableRef {
@@ -346,6 +347,99 @@ __global__ void index_apply_seq_kernel(TableRef t, const OpRec* __restrict__ ops
                                        unsigned long long scan_max_slots) {
   if (blockIdx.x != 0 || threadIdx.x != 0) return;
   apply_seq(t, ops, ents, start, n, seq_base, max_keys, order_ts, order_slot, order_n, scan_max_slots);
+}
+
+// ---- pod removal (kvb_index_remove_pods): one sweep over every slot.  No reference counterpart: the reference ignores
+// AllBlocksCleared (pool.go:388-395) and only removes a pod through Evict of keys the caller names.
+struct TierMask {  // 256 device tiers, one bit each; travels in the kernel arguments
+  uint32_t bits[8];
+};
+
+// One bucket: drop every entry whose pod is in `pod_bits` and whose tier is in `tiers` (the speculative bit is not
+// looked at), keep the rest in their inner-LRU order and write the bucket back only if it changed.  A key left empty is
+// deleted, as evictPodsFromRequestKey does (in_memory.go:281-292).  The recency stamp of a surviving key is NOT touched.
+// Returns the entries removed; *deleted = the key was deleted.
+KVB_DEV inline uint32_t purge_bucket(const TableRef& t, int64_t slot, uint32_t meta, const uint32_t* ent,
+                                     const uint32_t* __restrict__ pod_bits, const TierMask& tiers, bool* deleted) {
+  *deleted = false;
+  if ((meta & 3u) != kFull) return 0u;
+  const int raw_cnt = (int)((meta >> 8) & 0xffu), cnt = raw_cnt < kMaxEnt ? raw_cnt : kMaxEnt;
+  uint32_t keep[kMaxEnt];
+  int n = 0;
+#pragma unroll
+  for (int e = 0; e < kMaxEnt; ++e) keep[e] = 0u;
+#pragma unroll
+  for (int e = 0; e < kMaxEnt; ++e) {
+    if (e >= cnt) break;
+    const uint32_t v = ent[e], pod = v & 0xffffu, tier = (v >> 16) & 0xffu;
+    if (((pod_bits[pod >> 5] >> (pod & 31u)) & 1u) && ((tiers.bits[tier >> 5] >> (tier & 31u)) & 1u)) continue;
+#pragma unroll
+    for (int j = 0; j <= e; ++j)  // static indices: keep[] stays in registers
+      if (j == n) keep[j] = v;
+    ++n;
+  }
+  if (n == cnt) return 0u;
+  if (n == 0) {
+    kill_slot(t, slot);
+    *deleted = true;
+  } else {
+    store_bucket(t, slot, 0ull, keep, n, false);
+  }
+  return (uint32_t)(cnt - n);
+}
+
+KVB_DEV __forceinline__ void load_bucket(const Bucket* b, uint32_t* meta, uint32_t* ent) {
+#ifndef KVB_HOST_SIM
+  const uint4* src = reinterpret_cast<const uint4*>(b);  // key | meta ent0 | ent1-4 | ent5-8 | ent9-12
+  const uint4 q0 = src[0], q1 = src[1], q2 = src[2], q3 = src[3];
+  *meta = q0.z;
+  ent[0] = q0.w;
+  ent[1] = q1.x, ent[2] = q1.y, ent[3] = q1.z, ent[4] = q1.w;
+  ent[5] = q2.x, ent[6] = q2.y, ent[7] = q2.z, ent[8] = q2.w;
+  ent[9] = q3.x, ent[10] = q3.y, ent[11] = q3.z, ent[12] = q3.w;
+#else
+  *meta = b->meta;
+  for (int e = 0; e < kMaxEnt; ++e) ent[e] = b->ent[e];
+#endif
+}
+
+// Persistent grid, grid-stride over the slots, kPurgeUnroll buckets per thread per step: their 64 B loads are all issued
+// before any is looked at, so every thread keeps 128 B in flight.  Counters are summed per warp and added once per warp.
+constexpr int kPurgeThreads = 256, kPurgeUnroll = 2;
+
+__global__ void __launch_bounds__(kPurgeThreads)
+    index_remove_pods_kernel(TableRef t, const uint32_t* __restrict__ pod_bits, TierMask tiers) {
+  const uint64_t n_slots = t.mask + 1;
+  const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+  uint32_t removed = 0u, deleted = 0u;
+  for (uint64_t s0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s0 < n_slots; s0 += stride * kPurgeUnroll) {
+    uint32_t meta[kPurgeUnroll], ent[kPurgeUnroll][kMaxEnt];
+#pragma unroll
+    for (int u = 0; u < kPurgeUnroll; ++u) {
+      const uint64_t s = s0 + (uint64_t)u * stride;
+      meta[u] = kEmpty;
+      if (s < n_slots) load_bucket(&t.table[s], &meta[u], ent[u]);
+    }
+#pragma unroll
+    for (int u = 0; u < kPurgeUnroll; ++u) {
+      bool del = false;
+      removed += purge_bucket(t, (int64_t)(s0 + (uint64_t)u * stride), meta[u], ent[u], pod_bits, tiers, &del);
+      deleted += del ? 1u : 0u;
+    }
+  }
+#ifndef KVB_HOST_SIM
+  removed = __reduce_add_sync(0xffffffffu, removed);
+  deleted = __reduce_add_sync(0xffffffffu, deleted);
+  if ((threadIdx.x & 31) != 0) return;
+#endif
+  if (removed == 0u) return;
+  Counters& c = *t.ctr;
+  atomicAdd(&c.purge_entries, (unsigned long long)removed);
+  if (deleted == 0u) return;
+  atomicAdd(&c.purge_keys, (unsigned long long)deleted);
+  atomicAdd(&c.live, (unsigned long long)(-(long long)deleted));
+  atomicAdd(&c.tombs, (unsigned long long)deleted);
+  atomicAdd(&c.removed, (unsigned long long)deleted);
 }
 
 __global__ void index_sort_keys_kernel(const OpRec* __restrict__ ops, int64_t n, uint64_t* __restrict__ keys,
@@ -776,6 +870,7 @@ struct kvb_index {
   uint8_t* h_scratch_dev = nullptr;  // device alias of the pinned staging block (taken once, when it is allocated)
   size_t h_scratch_cap = 0;
   uint32_t* d_filter = nullptr;  // 65536 bits
+  uint32_t* d_purge_bits = nullptr;  // 65536 bits: the pods of the running kvb_index_remove_pods
   unsigned* d_done = nullptr;                 // prompts finished in the running fused launch (the kernel resets it)
   unsigned long long* h_done = nullptr;       // pinned word the last prompt writes the call's sequence number to
   unsigned long long done_seq = 0;
@@ -860,6 +955,8 @@ struct kvb_index {
   int flush_piece(size_t first, size_t count, bool may_evict);
   int queue_ops(uint8_t type, const uint64_t* keys, int64_t n_keys, const kvb_pod_entry_t* entries, int32_t n_entries);
   int set_filter(const uint16_t* pods, int32_t n, uint8_t* h_stage, bool* staged, const uint32_t** out);
+  int remove_pods_locked(const uint16_t* pods, int32_t n_pods, const uint8_t* tiers, int32_t n_tiers,
+                         int64_t* entries_removed, int64_t* keys_deleted);
 };
 
 int kvb_index::rehash(uint64_t new_slots) {
@@ -1280,6 +1377,44 @@ int kvb_index::set_filter(const uint16_t* pods, int32_t n, uint8_t* h_stage, boo
   return KVB_OK;
 }
 
+// kvb_index_remove_pods under the lock: queued ops first, then one sweep of the table.  Deleting keys turns live slots
+// into tombstones (live + tombs stays put), so no rehash is due here; flush_locked's growth rule stays the only one.
+int kvb_index::remove_pods_locked(const uint16_t* pods, int32_t n_pods, const uint8_t* tiers, int32_t n_tiers,
+                                  int64_t* entries_removed, int64_t* keys_deleted) {
+  int rc = flush_locked();
+  if (rc) return rc;
+  constexpr size_t kBitsBytes = 2048 * sizeof(uint32_t);
+  rc = ensure_scratch(0, kBitsBytes);
+  if (rc) return rc;
+  if (!d_purge_bits) KVB_CUDA_TRY(cudaMalloc(&d_purge_bits, kBitsBytes));
+  uint32_t* bits = reinterpret_cast<uint32_t*>(h_scratch);
+  std::memset(bits, 0, kBitsBytes);
+  for (int32_t i = 0; i < n_pods; ++i) bits[pods[i] >> 5] |= 1u << (pods[i] & 31);
+  TierMask tm;
+  std::memset(&tm, n_tiers > 0 ? 0 : 0xff, sizeof(tm));
+  for (int32_t i = 0; i < n_tiers; ++i) tm.bits[tiers[i] >> 5] |= 1u << (tiers[i] & 31);
+  KVB_CUDA_TRY(cudaMemcpyAsync(d_purge_bits, bits, kBitsBytes, cudaMemcpyHostToDevice, stream));
+  KVB_CUDA_TRY(cudaMemsetAsync(&d_ctr->purge_entries, 0, 2 * sizeof(unsigned long long), stream));
+  const uint64_t per_block = (uint64_t)kPurgeThreads * kPurgeUnroll;
+  uint64_t grid = (slots + per_block - 1) / per_block;
+#ifndef KVB_HOST_SIM
+  static int blocks_per_sm = 0;
+  if (blocks_per_sm == 0)
+    KVB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, index_remove_pods_kernel, kPurgeThreads, 0));
+  grid = std::min<uint64_t>(grid, (uint64_t)sm_count(device) * (uint64_t)std::max(blocks_per_sm, 1));
+#endif
+  KVB_LAUNCH(index_remove_pods_kernel, (unsigned)grid, kPurgeThreads, stream, ref(), d_purge_bits, tm);
+  KVB_CUDA_TRY(cudaGetLastError());
+  count_launch();
+  rc = sync_counters();  // live_ub / tomb_ub exact again
+  if (rc) return rc;
+  // the LRU order array is rebuilt the next time the index is at capacity; its records of freed slots are stale anyway
+  if (h_ctr.purge_keys) order_valid = false;
+  if (entries_removed) *entries_removed = (int64_t)h_ctr.purge_entries;
+  if (keys_deleted) *keys_deleted = (int64_t)h_ctr.purge_keys;
+  return KVB_OK;
+}
+
 // engineKey -> requestKeys mapping of one Add (in_memory.go:166-177): ek = engine[i*|E|/n], rk = request[i*|R|/n], n = max
 static void map_engine_keys(EngMap& em, const uint64_t* engine_keys, int64_t n_engine, const uint64_t* request_keys,
                             int64_t n_request) {
@@ -1395,7 +1530,7 @@ void kvb_index_destroy(kvb_index_t* idx) {
                   (void*)idx->d_sidx_out, idx->d_sort_tmp, (void*)idx->order_ts, (void*)idx->order_slot,
                   (void*)idx->order_ts_in, (void*)idx->order_slot_in, (void*)idx->d_cursor, (void*)idx->d_scratch,
                   (void*)idx->d_filter, (void*)idx->d_done, (void*)idx->d_plan_ops, (void*)idx->d_victims,
-                  (void*)idx->d_win, (void*)idx->d_plan, (void*)idx->d_conflict})
+                  (void*)idx->d_win, (void*)idx->d_plan, (void*)idx->d_conflict, (void*)idx->d_purge_bits})
     if (p) cudaFree(p);
   for (void* p : {(void*)idx->h_ops, (void*)idx->h_ents, (void*)idx->h_scratch, (void*)idx->h_done})
     if (p) cudaFreeHost(p);
@@ -1456,6 +1591,19 @@ int kvb_index_evict(kvb_index_t* idx, uint64_t key, int key_type, const kvb_pod_
     if (key_type == KVB_KEY_REQUEST) return idx->queue_ops(kOpEvict, &key, 1, entries, n_entries);
     set_error("unknown key type: %d", key_type);  // in_memory.go:252-254
     return KVB_ERR_INVALID;
+  });
+}
+
+int kvb_index_remove_pods(kvb_index_t* idx, const uint16_t* pods, int32_t n_pods, const uint8_t* tiers, int32_t n_tiers,
+                          int64_t* out_entries_removed, int64_t* out_keys_deleted) {
+  return kvb::guarded([&]() -> int {
+    KVB_REQUIRE(idx != nullptr, "index is NULL");
+    KVB_REQUIRE(n_pods >= 1 && pods, "no pods provided for removal from index");
+    KVB_REQUIRE(n_tiers >= 0 && (n_tiers == 0 || tiers), "bad tier list");
+    if (!tiers) n_tiers = 0;
+    std::lock_guard<std::mutex> lk(idx->mu);
+    DeviceGuard g(idx->device);
+    return idx->remove_pods_locked(pods, n_pods, tiers, n_tiers, out_entries_removed, out_keys_deleted);
   });
 }
 
@@ -1521,6 +1669,11 @@ int kvb_index_ingest_events(kvb_index_t* idx, const kvb_kv_event_t* ev, int32_t 
               if (rc) return rc;
             }
           }
+          continue;
+        }
+        if (x.type == KVB_EVENT_POD_CLEARED) {  // opt-in AllBlocksCleared: ops queued so far first, then the sweep
+          int rc = idx->remove_pods_locked(&x.entry.pod, 1, &x.entry.tier, 1, nullptr, nullptr);
+          if (rc) return rc;
           continue;
         }
         if (x.type != KVB_EVENT_BLOCK_STORED) continue;  // AllBlocksCleared and unknown events: log only (pool.go:388-395)

@@ -318,6 +318,25 @@ class Index:
             raise ValueError(f"unknown key type: {key_type}")
         self._check(self._lib.kvb_index_evict(self._h, int(key), int(key_type), self._entries(entries), len(entries)))
 
+    def remove_pods(self, pod_identifiers: Iterable[str], device_tiers: Optional[Iterable[str]] = None):
+        """Remove every entry of these pods (of these tiers; None = every tier) from every key, in one device sweep
+        (kvb_index_remove_pods).  Keys left empty are deleted; no key's recency changes; the engine-key map is untouched.
+        Names the index has never seen match nothing and are not interned.  Returns (entries_removed, keys_deleted)."""
+        pods = [self.pods.ids[n] for n in dict.fromkeys(pod_identifiers) if n in self.pods.ids]
+        tiers = None
+        if device_tiers is not None:
+            tiers = [self.tiers.ids[t] for t in dict.fromkeys(device_tiers) if t in self.tiers.ids]
+            if not tiers:
+                return 0, 0
+        if not pods:
+            return 0, 0
+        p = np.asarray(pods, dtype=np.uint16)
+        t = None if tiers is None else np.asarray(tiers, dtype=np.uint8)
+        removed, deleted = C.c_int64(), C.c_int64()
+        self._check(self._lib.kvb_index_remove_pods(self._h, p.ctypes.data, p.size, None if t is None else t.ctypes.data,
+                                                    0 if t is None else t.size, C.byref(removed), C.byref(deleted)))
+        return int(removed.value), int(deleted.value)
+
     def get_request_key(self, engine_key: int) -> int:
         out = C.c_uint64()
         rc = self._lib.kvb_index_get_request_key(self._h, int(engine_key), C.byref(out))

@@ -164,10 +164,14 @@ def realign_extra_features(engine_features, canonical_block_count: int):
 class EventProcessor:
     """Pool.processEventBatch (pool.go:253-398) over a kvblock.Index and a ChunkedTokenDatabase."""
 
-    def __init__(self, index: K.Index, token_processor: K.ChunkedTokenDatabase):
+    def __init__(self, index: K.Index, token_processor: K.ChunkedTokenDatabase, clear_on_all_blocks_cleared: bool = False):
         self.index = index
         self.token_processor = token_processor
         self.skipped = 0  # events the reference would log-and-continue on
+        # AllBlocksCleared: the reference only logs it (pool.go:388-395), so a pod that reset its prefix cache keeps
+        # attracting requests until the outer LRU pushes its entries out.  True: remove the pod's entries of the event's
+        # tier from the whole index (Index.remove_pods).
+        self.clear_on_all_blocks_cleared = bool(clear_on_all_blocks_cleared)
 
     # -- helpers -----------------------------------------------------------------------------------------------
     @staticmethod
@@ -204,6 +208,10 @@ class EventProcessor:
         for h in ev.block_hashes:  # pool.go:379-386
             self.index.evict(int(h), K.ENGINE_KEY, entries)
 
+    def _apply_cleared(self, ev, pod):
+        if self.clear_on_all_blocks_cleared:
+            self.index.remove_pods([pod], [self._tier(ev)])
+
     # -- reference-shaped entry point -------------------------------------------------------------------------
     def process_event_batch(self, batch, pod_identifier: str, model_name: str) -> None:
         events = batch.events if isinstance(batch, EventBatch) else batch
@@ -218,7 +226,8 @@ class EventProcessor:
                 self._apply_stored(ev, pod_identifier, keys or [])
             elif isinstance(ev, BlockRemovedEvent):
                 self._apply_removed(ev, pod_identifier)
-            # AllBlocksCleared / unknown: log only (pool.go:388-395)
+            elif isinstance(ev, AllBlocksClearedEvent):
+                self._apply_cleared(ev, pod_identifier)  # by default log only, as the reference (pool.go:388-395)
 
     def process_raw_message(self, adapter: VLLMAdapter, topic: str, payload: bytes) -> None:
         """Pool.processRawMessage (pool.go:196-204): parse failures are logged and dropped."""
@@ -267,6 +276,11 @@ class EventProcessor:
                     r.root_hash = tp.get_init_hash(ev.lora_name if ev.lora_name else model)  # pool.go:271-274
                 elif isinstance(ev, BlockRemovedEvent):
                     r.type = _lib.EVENT_BLOCK_REMOVED
+                elif isinstance(ev, AllBlocksClearedEvent) and self.clear_on_all_blocks_cleared:
+                    r.type = _lib.EVENT_POD_CLEARED
+                    r.entry.pod = idx.pods.get(pod)
+                    r.entry.tier = idx._tier_id(self._tier(ev))
+                    continue
                 else:
                     r.type = _lib.EVENT_OTHER
                     continue
@@ -308,6 +322,9 @@ class EventProcessor:
                     progressed = True
                     if isinstance(ev, BlockRemovedEvent):
                         self._apply_removed(ev, pod)
+                        continue
+                    if isinstance(ev, AllBlocksClearedEvent):
+                        self._apply_cleared(ev, pod)
                         continue
                     if isinstance(ev, BlockStoredEvent):
                         prep = self._prepare_stored(ev, model)
